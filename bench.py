@@ -11,6 +11,7 @@ frames (NN field + propagation) + CFG + DDIM update.  frames/s = N / (n_steps * 
   python bench.py --config {C2,C3,C4,C5s4,C5s8,C5s16}        the other BASELINE.json configs
   python bench.py --verify                                   + N-rank vs 1-rank (and graph vs eager) result check
   python bench.py --impl reference ...                       the reference's algorithm on host cores
+  python bench.py --dump-outputs DIR                         + DIR/latents.npy: what the last timed step returned
 
 One JSON line on stdout (rank 0).  Keys follow the driver contract; `roofline` describes the dominant hot-path
 kernel (per-launch CUDA events inside the timed region: event-record nodes of the captured step graphs, max over
@@ -128,6 +129,17 @@ class ClockSampler:
         sm.sort()
         return {"sm_mhz": sm[len(sm) // 2] if sm else None, "sm_max_mhz": max(smax) if smax else None,
                 "power_w_max": max(power) if power else None, "samples": len(sm), "reasons": sorted(reasons)}
+
+
+def dump_outputs(out_dir, arrays, limit=64 << 20):
+    """Write each array as <out_dir>/<name>.npy in float32, for comparing two builds output for output."""
+    import numpy as np
+    host = {name: t.detach().float().cpu().numpy() for name, t in arrays.items()}
+    total = sum(a.nbytes for a in host.values())
+    assert total <= limit, f"outputs are {total} bytes, more than {limit}"
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def dist_env():
@@ -323,6 +335,9 @@ def run_ours(args):
     ops.enable_timing(False)
     clocks = sampler.stop() if rank == 0 else None
     finite = bool(torch.isfinite(x.float()).all().item())
+    if args.dump_outputs and rank == 0:
+        # the denoised latents of every frame (all-gathered when sharded), as the step returns them to its caller
+        dump_outputs(args.dump_outputs, {"latents": x})
 
     # ---- end-to-end through the public call with pinned host latents (`e2e`) ----
     ms_e2e = float("nan")
@@ -673,7 +688,12 @@ def main():
                     help="1: one UNet call per step and GPU ([pivotal samples | frames], keyframe caches filled and "
                          "consumed inside each block); 0: the reference's pivotal pass + frame passes")
     ap.add_argument("--cudnn-benchmark", type=int, default=1, help="torch.backends.cudnn.benchmark for the UNet body convs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the latents the last timed step returned as DIR/latents.npy "
+                         "(float32; the inputs depend only on the arguments)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours: the reference arm times samples of a step and returns no latents")
     if not args.fused_pass:
         args.graph = 0                                   # graphs capture the fused step only
     if args.impl == "reference":

@@ -1,9 +1,8 @@
-"""ORACLE (test infrastructure) — import the UNMODIFIED reference hooks from /root/reference.
+"""ORACLE (test infrastructure) — import the UNMODIFIED reference hooks and drivers from the reference tree.
 
-Only usable in the build container (the GPU box has no /root/reference); used by
-`oracle/gen_golden.py` to produce `tests/golden/*.pt` and by `tests/test_reference_live.py`
-(skipped when the reference tree is absent).  Nothing is copied: the reference files are imported
-from where they lie.
+Only usable where the reference tree exists (TOKENFLOW_REFERENCE_DIR); used by `oracle/gen_golden.py`
+to produce `tests/golden/`, which the tests compare against.  Nothing is copied: the reference files
+are imported from where they lie.
 
 Why a shim is needed (SURVEY.md §8c): reference util.py:8 imports torchvision.io.read_video /
 write_video (removed in torchvision 0.26) and util.py:14-15 import kornia (not installed).
@@ -72,3 +71,31 @@ def load_reference():
         else:
             del sys.modules["util"]
     return ref_tf, ref_util
+
+
+def load_driver(filename: str, scheduler_cls):
+    """Import a reference driver (run_tokenflow_pnp.py / run_tokenflow_sdedit.py) with its `tokenflow_utils`
+    and `util` imports resolving to this repo's top-level drop-in modules.  `diffusers` is not installed: a
+    stub supplies `scheduler_cls` as its DDIMScheduler and an empty StableDiffusionPipeline (the driver's
+    __init__, which loads Stable Diffusion, is never run)."""
+    if not reference_available():
+        raise FileNotFoundError(f"reference tree not found at {REFERENCE_DIR}")
+    import tokenflow_utils as dropin_tf
+    import util as dropin_util
+    stub = types.ModuleType("diffusers")
+    stub.DDIMScheduler = scheduler_cls
+    stub.StableDiffusionPipeline = type("StableDiffusionPipeline", (), {})
+    saved = {k: sys.modules.get(k) for k in ("diffusers", "tokenflow_utils", "util")}
+    sys.modules.update({"diffusers": stub, "tokenflow_utils": dropin_tf, "util": dropin_util})
+    try:
+        name = "_ref_driver_" + filename.replace(".py", "")
+        spec = importlib.util.spec_from_file_location(name, os.path.join(REFERENCE_DIR, filename))
+        mod = importlib.util.module_from_spec(spec)
+        spec.loader.exec_module(mod)             # `if __name__ == '__main__'` does not fire
+    finally:
+        for k, v in saved.items():
+            if v is None:
+                sys.modules.pop(k, None)
+            else:
+                sys.modules[k] = v
+    return mod

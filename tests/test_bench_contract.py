@@ -42,3 +42,14 @@ def test_measured_peaks_and_env():
     p = bench.measured_peaks()
     assert p["hbm_gbs"] > 1000 and p["tf_sustained"] > 100 and p["source"] in ("measured", "fallback")
     assert bench.dist_env() == (0, 0, 1) or len(bench.dist_env()) == 3
+
+
+def test_dump_outputs_writes_float32_npy(tmp_path):
+    import numpy as np
+    import torch
+    x = torch.randn(2, 4, 8, 8).half()
+    bench.dump_outputs(str(tmp_path / "out"), {"latents": x})
+    a = np.load(tmp_path / "out" / "latents.npy")
+    assert a.dtype == np.float32 and np.array_equal(a, x.float().numpy())
+    with pytest.raises(AssertionError):
+        bench.dump_outputs(str(tmp_path / "big"), {"latents": x}, limit=100)

@@ -9,11 +9,10 @@ deviation is inside a *tie class*: two candidates whose fp16 similarity differs 
 where the winner depends on the fp32 accumulation order of the GEMM (cuBLAS's own order is not
 specified either).  Such rows are counted, bounded, and every one of them is checked.
 """
-import os
-
 import pytest
 import torch
 
+from oracle import golden
 from oracle import tokenflow_oracle as O
 from oracle.oracle_ops import OracleOps
 
@@ -24,10 +23,6 @@ pytestmark = pytest.mark.gpu
 def ops():
     from tokenflow_b200.ops import CudaOps
     return CudaOps()
-
-
-def _load(golden_dir, name):
-    return torch.load(os.path.join(golden_dir, name), weights_only=False)
 
 
 def _video_like(F, K, S, dim, seed, noise=0.3, device="cuda"):
@@ -281,7 +276,7 @@ def test_ext_attn_peaky_softmax(ops):
 
 def test_ext_attn_golden(ops, golden_dir):
     """Golden vectors of the unmodified reference (fp32 CPU) through the CUDA kernel (fp16)."""
-    for c in _load(golden_dir, "ext_attn.pt"):
+    for c in golden.load_ext_attn(golden_dir):
         q, k, v = (c[t].cuda().half() for t in ("q", "k", "v"))
         scale = (c["dim"] // c["heads"]) ** -0.5
         o = ops.ext_attn(q, k, v, c["heads"], scale, c["inject"]).float().cpu()

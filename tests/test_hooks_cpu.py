@@ -7,6 +7,7 @@ import pytest
 import torch
 import torch.nn as nn
 
+from oracle import golden
 from oracle.oracle_ops import OracleOps
 from tokenflow_b200 import sd_unet
 from tokenflow_b200 import tokenflow_utils as tfu
@@ -61,7 +62,7 @@ def test_no_fallback_without_gpu():
 
 def test_attention_closure_matches_reference(golden_dir):
     tfu._install_ops_for_testing(OracleOps())
-    for c in _load(golden_dir, "ext_attn.pt"):
+    for c in golden.load_ext_attn(golden_dir):
         block = sd_unet.BasicTransformerBlock(c["dim"], c["heads"], c["dim"] // c["heads"], 32).eval()
         block.attn1.load_state_dict(c["state_dict"])
         model = _Wrap(_OneBlockUNet(block))
@@ -77,7 +78,7 @@ def test_attention_closure_matches_reference(golden_dir):
 
 def test_tokenflow_block_matches_reference(golden_dir):
     tfu._install_ops_for_testing(OracleOps())
-    c = _load(golden_dir, "block_passes.pt")
+    c = golden.load_block_passes(golden_dir)
     block = sd_unet.BasicTransformerBlock(c["dim"], c["heads"], c["dim"] // c["heads"], c["ctx"]).eval()
     block.load_state_dict(c["state_dict"])
     model = _Wrap(_OneBlockUNet(block))
@@ -104,7 +105,7 @@ def test_tokenflow_block_matches_reference(golden_dir):
 def test_frame_table_equals_batch_idx(golden_dir):
     """register_frame_table (per-frame keyframes/weights) reproduces register_batch_idx."""
     tfu._install_ops_for_testing(OracleOps())
-    c = _load(golden_dir, "block_passes.pt")
+    c = golden.load_block_passes(golden_dir)
     block = sd_unet.BasicTransformerBlock(c["dim"], c["heads"], c["dim"] // c["heads"], c["ctx"]).eval()
     block.load_state_dict(c["state_dict"])
     model = _Wrap(_OneBlockUNet(block))

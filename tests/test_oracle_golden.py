@@ -1,27 +1,22 @@
 """CPU tier: the oracle restatement against the golden vectors the UNMODIFIED reference produced
 (oracle/gen_golden.py), and against the independent numpy closed form."""
-import os
-
 import numpy as np
 import pytest
 import torch
 
 from oracle import closed_form as CF
+from oracle import golden
 from oracle import tokenflow_oracle as O
-
-
-def _load(golden_dir, name):
-    return torch.load(os.path.join(golden_dir, name), weights_only=False)
 
 
 @pytest.fixture(scope="module")
 def attn_cases(golden_dir):
-    return _load(golden_dir, "ext_attn.pt")
+    return golden.load_ext_attn(golden_dir)
 
 
 @pytest.fixture(scope="module")
 def block_case(golden_dir):
-    return _load(golden_dir, "block_passes.pt")
+    return golden.load_block_passes(golden_dir)
 
 
 def _to_out(case, o):

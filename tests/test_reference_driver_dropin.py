@@ -1,96 +1,57 @@
-"""CPU tier, build container only: the UNMODIFIED reference driver (`/root/reference/run_tokenflow_pnp.py`
-and `run_tokenflow_sdedit.py`, class `TokenFlow`) running on this repo's drop-in `tokenflow_utils` / `util`
-modules.  The driver's own `init_method`, `denoise_step` and `batched_denoise_step` are executed as they
-are; only `__init__` (Stable-Diffusion download, VAE, CLIP, video files) is bypassed, and `diffusers` —
-which is not installed — is a stub that is never called.  The result must equal the golden produced by the
-reference hooks (oracle/gen_golden.py), which proves both that the hooks are a drop-in under the reference's
-own caller and that `tokenflow_b200/editor.py` mirrors that caller.  The oracle ops stand in for the CUDA
-kernels here (no GPU in this tier)."""
-import importlib.util
+"""CPU tier: this repo's drop-in `tokenflow_utils` / `util` modules against the UNMODIFIED reference drivers
+(run_tokenflow_pnp.py and run_tokenflow_sdedit.py, class `TokenFlow`).  oracle/gen_golden.py ran the drivers'
+own `init_method` and `batched_denoise_step` on the drop-in hooks and stored in tests/golden/driver_protocol.json
+the names they import from the drop-ins and every call they make into the hooks, the UNet and the scheduler
+(oracle/protocol.py); their result equalled the golden produced by the reference hooks.  Here
+`tokenflow_b200/editor.py` must export what the drivers import, make the same calls in the same order on the
+same values, and reach the same result, which shows both that the hooks are a drop-in under the reference's own
+caller and that the editor mirrors that caller.  The oracle ops stand in for the CUDA kernels (no GPU here)."""
+import json
 import os
-import sys
-import types
 
 import pytest
 import torch
-import torch.nn as nn
 
-from oracle import ref_shim
+from oracle import protocol
 from oracle.oracle_ops import OracleOps
 from tokenflow_b200 import sd_unet
 from tokenflow_b200 import tokenflow_utils as tfu
-from tokenflow_b200.editor import synthetic_inputs, write_latents_dir
+from tokenflow_b200.editor import TokenFlowEditor, synthetic_inputs, write_latents_dir
 from tokenflow_b200.scheduler import DDIMScheduler
-
-pytestmark = pytest.mark.skipif(not ref_shim.reference_available(), reason="reference tree not present")
-
-
-def _load_driver(filename):
-    """Import a reference driver with `tokenflow_utils` / `util` resolving to this repo's drop-ins."""
-    import tokenflow_utils as dropin_tf          # top-level drop-in modules of this repo
-    import util as dropin_util
-    stub = types.ModuleType("diffusers")
-    stub.DDIMScheduler = DDIMScheduler
-    stub.StableDiffusionPipeline = type("StableDiffusionPipeline", (), {})
-    saved = {k: sys.modules.get(k) for k in ("diffusers", "tokenflow_utils", "util")}
-    sys.modules.update({"diffusers": stub, "tokenflow_utils": dropin_tf, "util": dropin_util})
-    try:
-        name = "_ref_driver_" + filename.replace(".py", "")
-        spec = importlib.util.spec_from_file_location(name, os.path.join(ref_shim.REFERENCE_DIR, filename))
-        mod = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(mod)             # `if __name__ == '__main__'` does not fire
-    finally:
-        for k, v in saved.items():
-            if v is None:
-                sys.modules.pop(k, None)
-            else:
-                sys.modules[k] = v
-    return mod
-
-
-def _make_driver(mod, c, tmp_path, mode):
-    cfg = dict(c["config"])
-    unet = sd_unet.build_unet("tiny", seed=c["seed"])
-    x, text, pnp, src = synthetic_inputs(cfg["n_frames"], c["latent"], unet.config.cross_attention_dim,
-                                         cfg["n_timesteps"], seed=c["seed"], ctx_len=c["ctx_len"])
-    lat_dir = write_latents_dir(str(tmp_path), src)
-    ed = mod.TokenFlow.__new__(mod.TokenFlow)
-    nn.Module.__init__(ed)
-    ed.config = {"batch_size": cfg["batch_size"], "guidance_scale": cfg["guidance_scale"], "n_frames": cfg["n_frames"],
-                 "n_timesteps": cfg["n_timesteps"]}
-    ed.device = "cpu"
-    ed.sd_version = "1.5"
-    ed.unet = unet
-    ed.scheduler = DDIMScheduler()
-    ed.scheduler.set_timesteps(cfg["n_timesteps"], device="cpu")
-    if mode == "sdedit":                          # run_tokenflow_sdedit.py:57
-        ed.scheduler.timesteps = ed.scheduler.timesteps[int(1 - cfg["start"] * cfg["n_timesteps"]):]
-    ed.latents_path = lat_dir
-    ed.text_embeds = text
-    ed.pnp_guidance_embeds = pnp
-    return ed, x, cfg
 
 
 @pytest.mark.parametrize("mode,driver,golden", [("pnp", "run_tokenflow_pnp.py", "unet_c1_pnp.pt"),
                                                 ("sdedit", "run_tokenflow_sdedit.py", "unet_c1_sdedit.pt")])
 def test_unmodified_reference_driver_on_dropin_hooks(mode, driver, golden, golden_dir, tmp_path):
     c = torch.load(os.path.join(golden_dir, golden), weights_only=False)
-    mod = _load_driver(driver)
-    assert mod.register_pivotal is tfu.register_pivotal          # `from tokenflow_utils import *` bound OUR hooks
+    with open(os.path.join(golden_dir, "driver_protocol.json")) as f:
+        want = json.load(f)[driver]
+    import tokenflow_utils as dropin_tf                          # top-level drop-in modules of this repo
+    import util as dropin_util
+    for name in want["imports"]["tokenflow_utils"]:
+        assert hasattr(dropin_tf, name), name
+    for name in want["imports"]["util"]:
+        assert callable(getattr(dropin_util, name, None)), name
+    for name in protocol.HOOKS:                                  # `from tokenflow_utils import *` binds OUR hooks
+        assert getattr(dropin_tf, name) is getattr(tfu, name), name
+
+    cfg = dict(c["config"])
+    assert cfg["mode"] == mode
+    unet = sd_unet.build_unet("tiny", seed=c["seed"])
+    x, text, pnp, src = synthetic_inputs(cfg["n_frames"], c["latent"], unet.config.cross_attention_dim,
+                                         cfg["n_timesteps"], seed=c["seed"], ctx_len=c["ctx_len"])
+    cfg["latents_path"] = write_latents_dir(str(tmp_path), src)   # the drivers read source latents from disk
+    rec = protocol.Recorder()
     tfu._install_ops_for_testing(OracleOps())
-    ed, x, cfg = _make_driver(mod, c, tmp_path, mode)
-    if mode == "pnp":                                            # run_tokenflow_pnp.py:253-256
-        ed.init_method(conv_injection_t=int(cfg["n_timesteps"] * cfg["pnp_f_t"]),
-                       qk_injection_t=int(cfg["n_timesteps"] * cfg["pnp_attn_t"]))
-    else:                                                        # run_tokenflow_sdedit.py:191-193
-        ed.init_method()
+    ed = TokenFlowEditor(unet, rec.watch_scheduler(DDIMScheduler()), rec.hooks(tfu), cfg, text, pnp)
+    rec.watch_unet(unet)
+    ed.init_method()
     assert [int(t) for t in ed.scheduler.timesteps] == c["timesteps"]
     torch.manual_seed(c["seed"])
-    indices = torch.arange(cfg["n_frames"])
-    import warnings
-    with warnings.catch_warnings():
-        warnings.simplefilter("ignore")                          # the driver's cuda autocast decorator on a CPU box
-        for i, t in enumerate(ed.scheduler.timesteps):           # the body of sample_loop (:266-267), VAE decode omitted
-            x = ed.batched_denoise_step(x, t, indices)
-            assert torch.allclose(x, c["steps"][i], atol=2e-4, rtol=1e-4), f"step {i}"
-    assert torch.allclose(x, c["out"], atol=2e-4, rtol=1e-4)
+    steps = []
+    out = ed.sample_loop(x, on_step=lambda i, t, z: steps.append(z.clone()))
+    protocol.assert_same(rec.events, want["events"])
+    assert len(steps) == len(c["steps"])
+    for i, (got, ref) in enumerate(zip(steps, c["steps"])):
+        assert torch.allclose(got, ref, atol=2e-4, rtol=1e-4), f"step {i}"
+    assert torch.allclose(out, c["out"], atol=2e-4, rtol=1e-4)

@@ -1,45 +1,42 @@
-"""CPU tier, build container only: the oracle against the UNMODIFIED reference hooks executed live
-on fresh seeds (skipped where /root/reference does not exist, e.g. the GPU box — there the
-committed golden vectors stand in)."""
+"""CPU tier: the oracle against outputs of the UNMODIFIED reference hooks and helpers on fresh seeds,
+stored in tests/golden/reference_live.pt by oracle/gen_golden.py (the reference's extended attention on
+small blocks, its batch_cosine_sim and isinstance_str)."""
+import os
+
 import pytest
 import torch
-import torch.nn as nn
 
-from oracle import ref_shim
 from oracle import tokenflow_oracle as O
 from tokenflow_b200 import sd_unet
 
-pytestmark = pytest.mark.skipif(not ref_shim.reference_available(), reason="reference tree not present")
+
+@pytest.fixture(scope="module")
+def live(golden_dir):
+    return torch.load(os.path.join(golden_dir, "reference_live.pt"), weights_only=False)
 
 
 @pytest.mark.parametrize("seed,n,S,dim,heads,pnp,inject", [
     (101, 2, 24, 32, 2, False, False), (102, 4, 20, 64, 4, True, True), (103, 4, 20, 64, 4, True, False),
     (104, 13, 8, 32, 4, True, True)])
-def test_live_extended_attention(seed, n, S, dim, heads, pnp, inject):
-    from oracle.gen_golden import _OneBlockUNet, _Wrap
-    ref, _ = ref_shim.load_reference()
-    torch.manual_seed(seed)
+def test_live_extended_attention(live, seed, n, S, dim, heads, pnp, inject):
+    c = live["attention"][seed]
+    assert (c["n"], c["S"], c["dim"], c["heads"], c["inject"]) == (n, S, dim, heads, inject)
     block = sd_unet.BasicTransformerBlock(dim, heads, dim // heads, 16).eval()
-    model = _Wrap(_OneBlockUNet(block))
-    if pnp:
-        ref.register_extended_attention_pnp(model, [981] if inject else [])
-        block.attn1.t = 981
-    else:
-        ref.register_extended_attention(model)
-    x = torch.randn(3 * n, S, dim)
+    block.attn1.load_state_dict(c["state_dict"])
+    x = c["x"]
     with torch.no_grad():
-        want = block.attn1(x)
         a = block.attn1
         got = a.to_out[0](O.extended_attention(a.to_q(x), a.to_k(x), a.to_v(x), heads, a.scale, inject))
-    assert torch.allclose(got, want, atol=2e-6, rtol=1e-5)
+    assert torch.allclose(got, c["out"], atol=2e-6, rtol=1e-5)
 
 
-def test_live_cosine_sim_and_isinstance_str():
-    _, ref_util = ref_shim.load_reference()
+def test_live_cosine_sim_and_isinstance_str(live):
     from tokenflow_b200.util import isinstance_str
-    torch.manual_seed(5)
-    x, y = torch.randn(50, 24), torch.randn(30, 24)
-    assert torch.equal(O.cosine_sim(x, y), ref_util.batch_cosine_sim(x, y))
+    cs = live["cosine_sim"]
+    # the same ops as the reference; bit-equal where the reference ran, and a BLAS built for another CPU
+    # may order the 24-term dot products differently
+    assert torch.allclose(O.cosine_sim(cs["x"], cs["y"]), cs["out"], atol=1e-6, rtol=0)
     blk = sd_unet.BasicTransformerBlock(16, 2, 8, 8)
-    for name in ("BasicTransformerBlock", "Module", "Attention", "object"):
-        assert isinstance_str(blk, name) == ref_util.isinstance_str(blk, name)
+    assert len(live["isinstance_str"]) == 4
+    for name, want in live["isinstance_str"].items():
+        assert isinstance_str(blk, name) == want
